@@ -187,10 +187,16 @@ class Runner(object):
         self.micro_items, self.spans = plan['micro_items'], plan['spans']
         self.comm = None            # dist.Comm: the all-gather through the C ABI (set by main for world > 1)
 
-    def forward_all(self):
-        last = None
+    def forward_all(self, keep=False):
+        """Every micro-batch of this rank's shard; returns the last one's outputs (views into the model's buffers).
+        keep: also hold a copy of every micro-batch's outputs, concatenated, in self.kept (--dump-outputs)."""
+        last, kept = None, []
         for (i, j) in self.spans:
             last = self.model.forward_device(self.x_dev[i:j])
+            if keep:
+                kept.append([o.clone() for o in last])
+        if keep:
+            self.kept = [self.torch.cat(parts) for parts in zip(*kept)]
         return last
 
     def exchange(self, outs, which):
@@ -205,12 +211,13 @@ class Runner(object):
         local = torch.stack([o for o in outs if o.dim() == 2], dim=1)    # action probabilities (B_local, n_pred, n_act)
         return gather_outputs(local.contiguous(), self.world, comm=self.comm)
 
-    def step(self, which):
-        return self.exchange(self.forward_all(), which)
+    def step(self, which, keep=False):
+        return self.exchange(self.forward_all(keep), which)
 
 
-def timed_steps(torch, dist, world, fn, steps, warmup):
-    """W warm-ups, then K steps bracketed by barrier + synchronize, CUDA events, max over ranks -> ms per step."""
+def timed_steps(torch, dist, world, fn, steps, warmup, last_fn=None):
+    """W warm-ups, then K steps bracketed by barrier + synchronize, CUDA events, max over ranks -> ms per step.
+    last_fn: run instead of fn as the last timed step."""
     def barrier():
         if world > 1:
             dist.barrier()
@@ -220,14 +227,36 @@ def timed_steps(torch, dist, world, fn, steps, warmup):
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
-        fn()
+    for i in range(steps):
+        (last_fn if last_fn is not None and i == steps - 1 else fn)()
     e1.record()
     barrier()
     t = torch.tensor([e0.elapsed_time(e1)], device='cuda')
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return float(t.item()) / steps
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, outs):
+    """The outputs of every micro-batch of this rank's shard in the last timed step, as DIR/out<i>.npy (float32, the
+    model's output order, items in input order), so that two builds can be compared output for output: the inputs and
+    weights are seeded, so the same arguments give the same inputs on every run.  Above DUMP_LIMIT_BYTES in all, every
+    array keeps the same fixed, seeded sample of its leading rows (DIR/rows.npy lists them)."""
+    arrays = [o.detach().float().cpu().numpy() for o in outs]
+    total = sum(a.nbytes for a in arrays)
+    os.makedirs(directory, exist_ok=True)
+    if total > DUMP_LIMIT_BYTES:
+        n = arrays[0].shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_LIMIT_BYTES // total), replace=False))
+        arrays = [a[rows] for a in arrays]
+        np.save(os.path.join(directory, 'rows.npy'), rows)
+    names = ['out%02d' % i for i in range(len(arrays))]
+    for name, a in zip(names, arrays):
+        np.save(os.path.join(directory, name + '.npy'), a)
+    return names
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -446,9 +475,14 @@ def main():
     ap.add_argument('--no-secondary', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='plain launches instead of CUDA-graph replays')
     ap.add_argument('--precision', type=int, default=3)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of every micro-batch of the last timed step (rank 0\'s shard) to DIR/out<i>.npy; '
+                         'that step also copies them on the device; above 64 MB, a fixed sample of rows')
     ap.add_argument('--emulate-world', type=int, default=0,
                     help='analysis only (1 GPU): run rank 0 shard of a W-GPU strong-scaling job without the exchange step')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -493,8 +527,13 @@ def main():
     model.launch_total = 0
     sampler = ClockSampler(local)
     sampler.start()
-    ms_step = timed_steps(torch, dist, world, lambda: run.step(which), args.steps, args.warmup)
+    ms_step = timed_steps(torch, dist, world, lambda: run.step(which), args.steps, args.warmup,
+                          last_fn=(lambda: run.step(which, keep=True)) if args.dump_outputs else None)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        note('outputs of the last timed step -> %s/{%s}.npy' % (args.dump_outputs, ','.join(
+            dump_outputs(args.dump_outputs, run.kept))))
+    run.kept = None
     launches = int(getattr(model, 'launch_total', 0)) * args.steps // max(1, args.steps + args.warmup)
     value = n_frames / (ms_step / 1000.0)
 

@@ -1,5 +1,5 @@
-"""Case table shared by make_reference_golden.py (which runs the REFERENCE builders on keras_shim) and
-tests/test_reference_golden.py (which checks the oracle and the product against the fixtures it wrote)."""
+"""Case tables shared by the golden generators (which run the REFERENCE builders on keras_shim or on the recording
+keras) and the tests that check the oracle and the product against the fixtures they wrote."""
 
 RECEPTION_CASES = {
     # case: (input shape, reception.build kwargs, weight seed, input seed[, frames])
@@ -73,3 +73,72 @@ MERGE_CASE = dict(input_shape=(64, 64, 3), num_frames=4, num_actions=15, num_joi
 # the PoseAR net pools and re-upsamples the joint axis, which only closes for joint counts divisible by 4
 MERGE3D_CASE = dict(input_shape=(64, 64, 3), num_frames=4, num_actions=15, num_joints=20, num_blocks=2, depth_maps=8, seed=9,
                     reception=dict(num_joints=20, dim=3, num_blocks=2, depth_maps=8, ksize=(5, 5)))
+
+
+# builder arguments the BASELINE configs do not use, recorded on the recording keras (reference_dropin/
+# run_reference_backbone.py sweep -> ref_dropin_models.json.gz; tests/test_keras_compat.py): reception.build at 128x128 ...
+RECORDED_SWEEP_RECEPTION = (
+    dict(dim=2, num_context_per_joint=None, num_blocks=1, ksize=(3, 3)),
+    dict(dim=2, num_context_per_joint=1, num_blocks=2, ksize=(5, 5), export_heatmaps=True),
+    dict(dim=2, num_context_per_joint=2, num_blocks=2, ksize=(3, 3), concat_pose_confidence=False, alpha=0.5,
+         export_vfeat_block=1),
+    dict(dim=3, depth_maps=8, num_blocks=2, ksize=(3, 3)),
+    dict(dim=3, num_blocks=1, ksize=(5, 5), export_heatmaps=True),         # refused by both
+    dict(dim=4, num_blocks=1))                                             # the reference's own ValueError
+# ... and spnet.build: (input shape, pose layout, ModelConfig kwargs over SWEEP_SPNET_BASE)
+SWEEP_SPNET_BASE = dict(num_pyramids=2, num_levels=4, num_actions=[15], action_pyramids=[1, 2])
+RECORDED_SWEEP_SPNET = (
+    ((128, 128, 3), 'pa16j2d', dict(num_actions=[], action_pyramids=[], num_levels=3)),
+    ((128, 128, 3), 'pa17j3d', dict(num_actions=[], action_pyramids=[], predict_rootz=True, growth=64)),
+    ((4, 128, 128, 3), 'pa16j2d', dict(pose_replica=True, kernel_size=(3, 3))),
+    ((4, 128, 128, 3), 'pa20j3d', dict(num_actions=[15, 60], sam_alpha=2)),
+    ((16, 128, 128, 3), 'pa17j3d', dict(action_pyramids=[2], image_div=4)),
+    ((16, 128, 128, 3), 'pa16j2d', dict(num_pyramids=3, action_pyramids=[1, 3], num_pose_features=160,
+                                        num_visual_features=96)),
+    ((4, 128, 128, 3), 'pa16j2d', dict(downsampling_type='conv')))         # transposed conv: refused by both
+
+# the same kind of options executed numerically on keras_shim (make_option_sweep_golden.py -> ref_option_sweep.npz;
+# tests/test_reference_golden.py): reception.build at 64x64 on 2 frames, spnet.build on one item; inputs are drawn in
+# this order from one default_rng(OPTION_SWEEP_INPUT_SEED), weights are the product's synthetic ones (seed 1234)
+OPTION_SWEEP_INPUT_SEED = 2020
+OPTION_SWEEP_RECEPTION = RECORDED_SWEEP_RECEPTION[:4]
+OPTION_SWEEP_SPNET = (
+    ((128, 128, 3), 'pa16j2d', dict(num_actions=[], action_pyramids=[], num_levels=3)),
+    ((128, 128, 3), 'pa17j3d', dict(num_actions=[], action_pyramids=[], predict_rootz=True, growth=64)),
+    ((4, 128, 128, 3), 'pa16j2d', dict(pose_replica=True, kernel_size=(3, 3))),
+    ((4, 128, 128, 3), 'pa20j3d', dict(num_actions=[15, 60], sam_alpha=2)),
+    ((8, 128, 128, 3), 'pa17j3d', dict(action_pyramids=[2], image_div=4)),
+    ((4, 128, 128, 3), 'pa16j2d', dict(num_pyramids=3, action_pyramids=[1, 3], num_pose_features=160,
+                                       num_visual_features=96)))
+
+
+def option_sweep_inputs():
+    """[(kind, build kwargs / (shape, layout, kwargs), x float64)] of the numeric option sweep, in drawing order."""
+    import numpy as np
+    rng = np.random.default_rng(OPTION_SWEEP_INPUT_SEED)
+    out = [('reception', kw, rng.uniform(-1, 1, (2, 64, 64, 3))) for kw in OPTION_SWEEP_RECEPTION]
+    for shape, layout, extra in OPTION_SWEEP_SPNET:
+        kw = dict(SWEEP_SPNET_BASE)
+        kw.update(extra)
+        out.append(('spnet', (shape, layout, kw), rng.uniform(-1, 1, (1,) + shape)))
+    return out
+
+
+OPTION_SWEEP_SAMPLE = 4096      # outputs with more elements are stored as this many values at fixed positions
+
+
+def option_sweep_sample_index(size):
+    """Positions (in the flattened output) of the values ref_option_sweep.npz keeps of a large output."""
+    import numpy as np
+    return np.sort(np.random.default_rng(0).choice(size, OPTION_SWEEP_SAMPLE, replace=False))
+
+
+def option_sweep_store(blob, key, out):
+    """Output `key` of the option sweep into `blob`: whole, or its shape and a fixed sample of its values."""
+    import numpy as np
+    out = np.asarray(out, dtype=np.float64)
+    if out.size <= OPTION_SWEEP_SAMPLE:
+        blob[key] = out
+    else:
+        blob[key + '_shape'] = np.array(out.shape)
+        blob[key + '_sample'] = out.ravel()[option_sweep_sample_index(out.size)]

@@ -1,6 +1,8 @@
 """Executes the reference's own model builders after deephar_b200.dropin.install() and prints the recorded model's
-weight list, kernel plan, output shapes and expression digests as JSON (driven by tests/test_keras_compat.py in a
-subprocess, only where the reference tree exists)."""
+weight list, kernel plan, output shapes and expression digests as JSON.  Runs where the reference tree exists
+(DEEPHAR_REFERENCE); tests/golden/make_dropin_golden.py stores what it prints for tests/test_keras_compat.py.
+
+    DEEPHAR_REFERENCE=<reference checkout> python run_reference_backbone.py <case>"""
 import json
 import os
 import sys
@@ -8,7 +10,9 @@ import warnings
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path[:0] = [os.environ.get('DEEPHAR_REFERENCE', '/root/reference'), ROOT]
+if not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '')):
+    raise SystemExit('set DEEPHAR_REFERENCE to the reference checkout')
+sys.path[:0] = [os.environ['DEEPHAR_REFERENCE'], ROOT]
 warnings.filterwarnings('ignore')
 import deephar_b200.dropin  # noqa: E402
 deephar_b200.dropin.install()                                 # `keras` / `tensorflow` -> the recording front end
@@ -107,62 +111,37 @@ def merge_model_case(pose_dim, version='v1'):
 
 
 def option_sweep_case():
-    """Builder options off the BASELINE configs: the reference's reception.build / spnet.build (unmodified, recorded) against
-    deephar_b200's builders for the same arguments -- weight lists, output expressions, output shapes, launches.  One JSON
-    line per configuration.  (spnet.py:210-214 keeps a module-level action-block counter across builds in one process --
-    a second model is named act7_..., which breaks by_name loading in the reference itself; reset here per build.)"""
+    """Builder options off the BASELINE configs (ref_cases.RECORDED_SWEEP_*): the reference's reception.build /
+    spnet.build (unmodified, recorded), one JSON line per configuration -- the recorded weight list, output expressions,
+    output shapes and launch kinds, or the exception the builder raised.  tests/test_keras_compat.py builds the product
+    model for the same arguments and compares.  (spnet.py:210-214 keeps a module-level action-block counter across builds
+    in one process -- a second model is named act7_..., which breaks by_name loading in the reference itself; reset here
+    per build.)"""
     from deephar.config import ModelConfig as RefConfig
     from deephar.models import spnet as S
     from deephar.utils import pose as ref_pose
-    from deephar_b200 import reception as PR
-    from deephar_b200 import spnet as PS
-    from deephar_b200 import config as pconfig
+    sys.path.insert(0, os.path.join(ROOT, 'tests', 'golden'))
+    from ref_cases import RECORDED_SWEEP_RECEPTION, RECORDED_SWEEP_SPNET, SWEEP_SPNET_BASE
 
-    def compare(tag, ref_fn, prod_fn):
+    def record(tag, ref_fn):
         keras_compat.clear_session()
         S.__dict__.pop('act_cnt', None)
         res = {'tag': tag}
         try:
             ref = ref_fn()
-            ref.weight_specs
+            res.update(weight_specs=[[n, list(s)] for n, s in ref.weight_specs], signatures=ref.graph.signatures(),
+                       output_shape=[list(s) for s in ref.output_shape], kinds=sorted(k.kind for k in ref.plan.kops))
         except Exception as e:                                  # noqa: BLE001
-            ref, res['ref_error'] = None, type(e).__name__
-        try:
-            prod = prod_fn()
-        except Exception as e:                                  # noqa: BLE001
-            prod, res['prod_error'] = None, type(e).__name__
-        if ref is not None and prod is not None:
-            res['weights'] = [(n, tuple(s)) for n, s in ref.weight_specs] == [(n, tuple(s)) for n, s in prod.weight_specs]
-            res['signatures'] = ref.graph.signatures() == prod.graph.signatures()
-            res['shapes'] = [tuple(s) for s in ref.output_shape] == [tuple(s) for s in prod.output_shape]
-            res['launches'] = sorted(k.kind for k in ref.plan.kops) == sorted(k.kind for k in prod.plan.kops)
-            res['n_launches'] = len(prod.plan.kops)
+            res = {'tag': tag, 'ref_error': type(e).__name__}
         print(json.dumps(res))
 
-    for kw in (dict(dim=2, num_context_per_joint=None, num_blocks=1, ksize=(3, 3)),
-               dict(dim=2, num_context_per_joint=1, num_blocks=2, ksize=(5, 5), export_heatmaps=True),
-               dict(dim=2, num_context_per_joint=2, num_blocks=2, ksize=(3, 3), concat_pose_confidence=False, alpha=0.5,
-                    export_vfeat_block=1),
-               dict(dim=3, depth_maps=8, num_blocks=2, ksize=(3, 3)),
-               dict(dim=3, num_blocks=1, ksize=(5, 5), export_heatmaps=True),         # refused by both
-               dict(dim=4, num_blocks=1)):                                            # the reference's own ValueError
+    for kw in RECORDED_SWEEP_RECEPTION:
         nj = 17 if kw.get('dim') == 3 else 16
-        compare('reception %r' % (kw,), lambda: R.build((128, 128, 3), nj, **kw), lambda: PR.build((128, 128, 3), nj, **kw))
-    base = dict(num_pyramids=2, num_levels=4, num_actions=[15], action_pyramids=[1, 2])
-    for shape, layout, extra in (
-            ((128, 128, 3), 'pa16j2d', dict(num_actions=[], action_pyramids=[], num_levels=3)),
-            ((128, 128, 3), 'pa17j3d', dict(num_actions=[], action_pyramids=[], predict_rootz=True, growth=64)),
-            ((4, 128, 128, 3), 'pa16j2d', dict(pose_replica=True, kernel_size=(3, 3))),
-            ((4, 128, 128, 3), 'pa20j3d', dict(num_actions=[15, 60], sam_alpha=2)),
-            ((16, 128, 128, 3), 'pa17j3d', dict(action_pyramids=[2], image_div=4)),
-            ((16, 128, 128, 3), 'pa16j2d', dict(num_pyramids=3, action_pyramids=[1, 3], num_pose_features=160,
-                                                num_visual_features=96)),
-            ((4, 128, 128, 3), 'pa16j2d', dict(downsampling_type='conv'))):           # transposed conv: refused by both
-        kw = dict(base)
+        record('reception %r' % (kw,), lambda: R.build((128, 128, 3), nj, **kw))
+    for shape, layout, extra in RECORDED_SWEEP_SPNET:
+        kw = dict(SWEEP_SPNET_BASE)
         kw.update(extra)
-        compare('spnet %r %s %r' % (shape, layout, extra),
-                lambda: S.build(RefConfig(shape, getattr(ref_pose, layout), **kw)),
-                lambda: PS.build(pconfig.ModelConfig(shape, getattr(pconfig, layout), **kw)))
+        record('spnet %r %s %r' % (shape, layout, extra), lambda: S.build(RefConfig(shape, getattr(ref_pose, layout), **kw)))
 
 
 def main():

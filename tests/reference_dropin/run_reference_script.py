@@ -20,10 +20,12 @@ eval_penn_multitask.py imports `eval_singleclip_generator`, which exp/common/pen
 `eval_singleclip_gt_bbox_generator` (the script fails with ImportError on the reference's own stack too).
 
 Prints one JSON line: every score an evaluator returned to the script, the same scores recomputed from the oracle's outputs
-alone, and what the compiled model looks like.
+alone (standins.py), what the compiled model looks like and, for h36m, the cameras and poses of the stand-in dataset.
+tests/golden/make_entry_script_golden.py stores it for tests/test_keras_compat.py.
+
+    DEEPHAR_REFERENCE=<reference checkout> python run_reference_script.py <case> <empty working directory>
 """
 import contextlib
-import hashlib
 import io
 import json
 import os
@@ -34,7 +36,9 @@ import warnings
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get('DEEPHAR_REFERENCE', '/root/reference')
+REF = os.environ.get('DEEPHAR_REFERENCE', '')
+if not os.path.isdir(REF):
+    raise SystemExit('set DEEPHAR_REFERENCE to the reference checkout')
 sys.path[:0] = [REF, ROOT]
 warnings.filterwarnings('ignore')
 import numpy as np  # noqa: E402
@@ -47,63 +51,13 @@ import deephar.data  # noqa: E402
 sys.stderr = _stderr
 
 from deephar_b200 import keras_h5  # noqa: E402
-from deephar_b200.compiler import verify_plan  # noqa: E402
 from deephar_b200 import model as product_model  # noqa: E402
-from deephar_b200 import reception as product_reception  # noqa: E402
-from deephar_b200 import spnet as product_spnet  # noqa: E402
-from deephar_b200.config import ModelConfig as ProductConfig  # noqa: E402
-from deephar_b200.config import pa16j2d as product_pa16j2d  # noqa: E402
-from deephar_b200.config import pa17j3d as product_pa17j3d  # noqa: E402
-from oracle import ops_torch, synth  # noqa: E402
 from oracle import postprocess as oracle_post  # noqa: E402
-from oracle import reception as oracle_reception  # noqa: E402
-from oracle import spnet as oracle_spnet  # noqa: E402
+sys.path.insert(0, HERE)
+from standins import (CASES, ClipDataset, N_FRAMES, Oracle, T, describe_script_model,  # noqa: E402
+                      expected_action_scores, expected_pckh, h36m_frames, mpii_batches, set_clip_labels)
 
 ON_GPU = os.environ.get('DEEPHAR_B200_SCRIPT_ON_GPU') == '1'
-T = 8                                   # num_frames of both multitask scripts
-
-PENN_KW = dict(num_actions=[15], num_pyramids=6, action_pyramids=[5, 6], num_levels=4, pose_replica=True,
-               num_pose_features=160, num_visual_features=160)
-NTU_KW = dict(num_actions=[60], num_pyramids=2, action_pyramids=[1, 2], num_levels=4, pose_replica=False,
-              num_pose_features=192, num_visual_features=192)
-CASES = {
-    'mpii': dict(script='exp/mpii/eval_mpii_singleperson.py', cache='weights_PE_MPII_cvpr18_19-09-2017.h5',
-                 reception=dict(num_joints=16, dim=2, num_blocks=8, num_context_per_joint=2, ksize=(5, 5),
-                                concat_pose_confidence=False)),
-    'h36m': dict(script='exp/h36m/eval_h36m.py', cache='weights_3DPE_H36M_cvpr18_Nov-2017.h5',
-                 reception=dict(num_joints=17, dim=3, num_blocks=8, ksize=(5, 5), concat_pose_confidence=False)),
-    'penn_multitask': dict(script='exp/pennaction/eval_penn_multitask.py', local='weights/weights_mpii+penn_ar_028.hdf5',
-                           spnet=(PENN_KW, product_pa16j2d, oracle_spnet.pa16j2d), action=('pennaction', 15)),
-    'ntu_multitask': dict(script='exp/ntu/eval_ntu_multitask.py',
-                          local='output/ntu_spnet_trial-03-ft_replica_0ae2bf7/weights_3dp+ntu_ar_062.hdf5',
-                          spnet=(NTU_KW, product_pa17j3d, oracle_spnet.pa17j3d), action=('ntuaction', 60)),
-}
-
-
-class Oracle(object):
-    """The CPU oracle's forward of the case's model: all outputs of the FULL model, as float32 arrays."""
-
-    def __init__(self, case):
-        self.case = case
-        if 'reception' in case:
-            self.model = product_reception.build((256, 256, 3), **case['reception'])
-        else:
-            kw, layout, olayout = case['spnet']
-            self.model = product_spnet.build(ProductConfig((T, 256, 256, 3), layout, **kw))
-            self.ocfg = oracle_spnet.ModelConfig((T, 256, 256, 3), olayout, **kw)
-        self.model.init_synthetic_weights(77)
-        self.table = self.model.get_weights()
-        self.memo = {}
-
-    def __call__(self, table, x):
-        key = (x.shape, hashlib.sha1(np.ascontiguousarray(x).tobytes()).hexdigest())
-        if key not in self.memo:
-            if 'reception' in self.case:
-                outs = oracle_reception.forward(ops_torch, table, x, **self.case['reception'])
-            else:
-                outs = oracle_spnet.forward(ops_torch, table, x, self.ocfg)
-            self.memo[key] = [np.asarray(o, np.float32) for o in outs]
-        return self.memo[key]
 
 
 def install_oracle_predict(oracle):
@@ -118,20 +72,11 @@ def install_oracle_predict(oracle):
     product_model.Model.predict = predict
 
 
-# ---- stand-ins for the datasets -------------------------------------------------------------------------------------
-def mpii_batches(n):
-    rng = np.random.default_rng(11)
-    x = synth.synth_frames(n, 256, 256, seed=21)
-    pose = np.concatenate([rng.uniform(0.2, 0.8, (n, 16, 2)), np.ones((n, 16, 1))], axis=-1)
-    afmat = np.tile(np.array([[1 / 300.0, 0, 0.05], [0, 1 / 300.0, 0.1], [0, 0, 1]]), (n, 1, 1))
-    head = rng.uniform(40, 60, (n, 1))
-    return [x], [pose, afmat, head]
-
-
+# ---- stand-ins for the datasets (the rest: standins.py) ---------------------------------------------------------
 def h36m_batches(n):
     from deephar.utils.camera import Camera
     rng = np.random.default_rng(36)
-    x = synth.synth_frames(n, 256, 256, seed=22)
+    x, afmat = h36m_frames(n)
     nj = 17
     scam, pose_w, uvd = [], np.zeros((n, nj, 3)), np.zeros((n, nj, 3))
     for i in range(n):
@@ -144,9 +89,6 @@ def h36m_batches(n):
         pts = np.concatenate([rng.normal(0, 400, (nj, 2)), rng.uniform(4000, 6000, (nj, 1))], axis=1)
         pose_w[i] = (np.matmul(cam.R_inv, pts.T) + cam.t).T
         uvd[i] = cam.project(pose_w[i])
-    afmat = np.zeros((n, 3, 3))
-    afmat[:, 0, 0] = afmat[:, 1, 1] = 1 / 500.0
-    afmat[:, 0, 2], afmat[:, 1, 2], afmat[:, 2, 2] = -0.3, -0.2, 1.0
     import deephar.data.human36m as h36m_data
     h36m_data.ACTION_LABELS = ['action%02d' % i for i in range(15)]      # set by the loader when it reads the annotations
     return [x], [pose_w, uvd, afmat, np.array(scam), rng.integers(0, 15, (n, 1))]
@@ -154,42 +96,13 @@ def h36m_batches(n):
 
 class FrameDataset(object):
     """MpiiSinglePerson / Human36M with topology='frames': only its length is asked for."""
-    n = 3
+    n = N_FRAMES
 
     def __init__(self, *args, **kwargs):
         pass
 
     def get_length(self, mode):
         return self.n
-
-
-class ClipDataset(object):
-    """PennAction / Ntu with topology='sequences': two test sequences of two clips each; the loader honours
-    `dataconf.fixed_hflip` as the real one does (deephar/data/pennaction.py:135-160)."""
-    key, n_actions, labels = 'pennaction', 15, (0, 0)
-
-    def __init__(self, path, dataconf, *args, **kwargs):
-        self.dataconf = dataconf
-        self.use_gt_bbox = kwargs.get('use_gt_bbox', True)
-
-    def get_length(self, mode):
-        return 2
-
-    def get_shape(self, key):
-        assert key == self.key
-        return (self.n_actions,)
-
-    def get_clip_index(self, i, mode, subsamples=[1]):
-        return [list(range(T)), list(range(3, 3 + T))]
-
-    def clip(self, i, start, hflip):
-        x = synth.synth_frames(T, 256, 256, seed=100 + 10 * i + start)
-        return x[:, :, ::-1].copy() if hflip else x
-
-    def get_data(self, i, mode, frame_list=None, bbox=None):
-        onehot = np.zeros(self.n_actions)
-        onehot[self.labels[i]] = 1
-        return {'frame': self.clip(i, frame_list[0], self.dataconf.fixed_hflip), self.key: onehot}
 
 
 def make_loader(frame_batches):
@@ -208,37 +121,6 @@ def make_loader(frame_batches):
             d = self.dataset.get_data(i, None, frame_list=[0])
             return [d['frame'][None]], [d[self.dataset.key][None]]
     return Loader
-
-
-# ---- the same scores from the oracle's outputs alone ----------------------------------------------------------------
-def expected_pckh(oracle, x, pose, afmat, head, n_pose_outputs, clip):
-    xin = x.reshape((-1, T) + x.shape[1:]) if clip else x
-    ref = oracle(oracle.table, xin)
-    y_true = oracle_post.transform_pose_sequence(afmat, pose[:, :, 0:2], inverse=True)
-    out = []
-    for b in range(n_pose_outputs):
-        p = ref[b if clip else 2 * b]
-        p = p.reshape((-1,) + p.shape[-2:])[:, :, 0:2]
-        out.append(oracle_post.pckh(y_true, oracle_post.transform_pose_sequence(afmat, p, inverse=True), head, 0.5))
-    return out
-
-
-def expected_action_scores(oracle, ds, first_action_output):
-    """exp/common/penn_tools.py:42-82 (single clip, accuracy as a fraction) and :85-150 / ntu_tools.py:53-140 (product
-    over clips x h-flip, accuracy in %)."""
-    n = ds.get_length(None)
-    single = [oracle(oracle.table, ds.clip(i, 0, 0)[None])[first_action_output:] for i in range(n)]
-    nb = len(single[0])
-    sc_single = [float(np.mean([np.argmax(single[i][b][0]) == ds.labels[i] for i in range(n)])) for b in range(nb)]
-    prod = np.ones((nb, n, ds.n_actions))
-    for i in range(n):
-        for fl in ds.get_clip_index(i, None):
-            for hflip in (0, 1):
-                pred = oracle(oracle.table, ds.clip(i, fl[0], hflip)[None])[first_action_output:]
-                for b in range(nb):
-                    prod[b, i] *= pred[b][0]
-    sc_multi = [float(100.0 * np.sum(np.argmax(prod[b], axis=-1) == np.array(ds.labels)) / n) for b in range(nb)]
-    return sc_single, sc_multi
 
 
 def main():
@@ -265,18 +147,7 @@ def main():
         FrameDataset.n = T                                      # the pose model of a clip network takes T frames at a time
     frames = h36m_batches(FrameDataset.n) if name == 'h36m' else mpii_batches(FrameDataset.n)
     if 'action' in case:
-        # ground truth: sequence 0 is labelled with what the last prediction block says about it (multi-clip product),
-        # sequence 1 with another class -- so that the accuracies are neither all 0 nor all 100
-        ClipDataset.key, ClipDataset.n_actions = case['action']
-        probe = ClipDataset(None, types.SimpleNamespace(fixed_hflip=0))
-        last = []
-        for i in range(2):
-            prod = np.ones(ClipDataset.n_actions)
-            for fl in probe.get_clip_index(i, None):
-                for hflip in (0, 1):
-                    prod = prod * oracle(oracle.table, probe.clip(i, fl[0], hflip)[None])[-1][0]
-            last.append(int(np.argmax(prod)))
-        ClipDataset.labels = (last[0], (last[1] + 1) % ClipDataset.n_actions)
+        set_clip_labels(oracle, case)
     for cls in ('MpiiSinglePerson', 'Human36M'):
         setattr(deephar.data, cls, FrameDataset)
     for cls in ('PennAction', 'Ntu'):
@@ -352,30 +223,15 @@ def main():
         else:
             want['eval_multiclip_dataset'] = [multi]
         model = action_model
-    impl = full._compiled()
-    held = impl.get_weights()
-    # the plan the script's final model compiled to, executed on the CPU on its own buffer layout (tests/plan_emulator.py),
-    # against the oracle's outputs for one item: pins the re-wired model's launch sequence, not only its scores
-    sys.path.insert(0, os.path.join(ROOT, 'tests'))
-    from plan_emulator import PlanEmulator
-    if name in ('mpii', 'h36m'):
-        x1 = frames[0][0][:1]
-        ref1 = oracle(oracle.table, x1)
-        ref1 = [np.concatenate([ref1[2 * b], ref1[2 * b + 1]], axis=-1) for b in range(len(ref1) // 2)]
-    else:
-        x1 = ds.clip(0, 0, 0)[None]
-        ref1 = oracle(oracle.table, x1)
-    with np.errstate(over='ignore'):
-        emu = PlanEmulator(impl).run(x1)
-    plan_err = max(float(np.abs(o - r).max()) for o, r in zip(emu, ref1))
-    assert len(emu) == len(ref1) and all(o.shape == r.shape for o, r in zip(emu, ref1))
+    model_desc, split = describe_script_model(name, oracle, full, [model] if name in ('mpii', 'h36m') else g['models'])
+    standin = {}
+    if name == 'h36m':
+        standin = {'pose_w': g['pw_val'].tolist(), 'uvd': g['puvd_val'].tolist(), 'scam': np.asarray(g['scam_val']).tolist()}
     print(json.dumps({
-        'returned': returned, 'oracle': {k: [[float(s) for s in v] for v in vs] for k, vs in want.items()},
+        'returned': returned, 'standin': standin, 'model': model_desc, 'split': split,
+        'oracle': {k: [[float(s) for s in v] for v in vs] for k, vs in want.items()},
         'model_class': type(model).__module__ + '.' + type(model).__name__, 'n_outputs': len(model.outputs),
-        'output_shape': [list(s) for s in model.output_shape],
-        'weights_are_the_files': set(held) == set(oracle.table) and all(np.array_equal(held[k], oracle.table[k])
-                                                                       for k in oracle.table),
-        'launches': len(impl.plan.kops), 'plan_emulation_max_err': plan_err, 'plan_checked': verify_plan(impl.plan, impl.graph), 'script_printed': printed.getvalue()[-600:],
+        'output_shape': [list(s) for s in model.output_shape], 'script_printed': printed.getvalue()[-600:],
         'forward': 'Model.predict' if ON_GPU else 'oracle (CPU stand-in)'}))
 
 

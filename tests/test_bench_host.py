@@ -70,7 +70,7 @@ def test_reference_arm_line_has_the_contract_keys(monkeypatch, capsys):
 
 @pytest.mark.timeout(600)
 @pytest.mark.parametrize('world', [1, 8])
-def test_bench_control_flow_on_the_stand_in_device(world):
+def test_bench_control_flow_on_the_stand_in_device(world, tmp_path):
     """bench.py from its first line to its JSON line on tests/fake_cuda.py (host memory as device memory, inert streams /
     events / graphs, gloo for NCCL, every device entry point of the C library a no-op): model builds, buffer binding,
     CUDA-graph branch, the copy-pipelined predict of the e2e leg, the per-kernel profile, the exchange step through
@@ -79,7 +79,8 @@ def test_bench_control_flow_on_the_stand_in_device(world):
     import socket
     import subprocess
     fake = os.path.join(ROOT, 'tests', 'fake_cuda.py')
-    tail = [fake, os.path.join(ROOT, 'bench.py'), '--gpus', str(world), '--steps', '1', '--warmup', '3', '--no-cpu-baseline']
+    tail = [fake, os.path.join(ROOT, 'bench.py'), '--gpus', str(world), '--steps', '1', '--warmup', '3', '--no-cpu-baseline',
+            '--dump-outputs', str(tmp_path / 'outs')]
     if world == 1:
         cmd = [sys.executable] + tail
     else:
@@ -103,6 +104,12 @@ def test_bench_control_flow_on_the_stand_in_device(world):
     assert d['e2e']['value'] > 0 and d['e2e']['h2d_bytes_per_step'] == 512 * 256 * 256 * 3 * 4 and d['e2e']['d2h_bytes_per_step'] > 0
     assert d['gpu_launches'] >= 127 * world and '127 kernels per forward' in d['launch_mode']
     assert set(d['roofline']) >= {'kernel', 'bound', 'achieved', 'peak', 'unit', 'frac', 'traffic'}
+    # the last timed step's outputs: per block (pose, visibility) of every frame of rank 0's shard -- both 256-frame
+    # forwards at N = 1
+    dumped = sorted(os.listdir(tmp_path / 'outs'))
+    assert dumped == ['out%02d.npy' % i for i in range(16)]
+    shapes = [np.load(tmp_path / 'outs' / f).shape for f in dumped]
+    assert shapes == [(512 // world, 16, 2), (512 // world, 16, 1)] * 8
     assert len(d['kernel_profile']) == 10 and 'cpu_baseline' not in d
     sec = d['secondary']
     assert set(sec) >= {'softargmax3d', 'input_pipeline', 'C1', 'C3', 'C4', 'C5'} and ('weak' in sec) == (world > 1)

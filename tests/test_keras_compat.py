@@ -1,6 +1,7 @@
 """keras_compat: model code written in the Keras functional style (the style of deephar/models/*.py) records the same
 graph, weight list and kernel plan as the function-style mirror of deephar/layers.py; unsupported Keras features are
 rejected when the model is built."""
+import gzip
 import json
 import os
 import subprocess
@@ -14,6 +15,10 @@ from deephar_b200 import layers as L
 from deephar_b200.graph import Graph
 from deephar_b200.model import Model
 from oracle import ops_torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+sys.path.insert(0, GOLDEN)
+sys.path.insert(0, os.path.dirname(GOLDEN))
 
 
 def _keras_style(inp):
@@ -160,17 +165,11 @@ def test_nested_models_and_session_counters():
         blk.predict(np.zeros((1, 16, 16, 8), np.float32))      # ... and then belongs to the outer model
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 def test_reference_backbone_builders_record_the_same_model():
     """The REFERENCE'S OWN code -- deephar/layers.py and models/reception.py::_stem / build_reception_block /
     build_sconv_block / build_regmap_block / build_fremap_block, unmodified -- imported on a `keras` that is
     keras_compat (tests/reference_dropin) records the weight list, auto-names and kernel plan of deephar_b200's builders."""
-    here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_backbone.py'), '3'],
-                         capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0, out.stderr[-2000:]
-    got = json.loads([l for l in out.stdout.splitlines() if l.startswith('{')][-1])
+    got = _recorded('3')
     want = _function_style_backbone(3)
     assert [(n, tuple(s)) for n, s in got['weight_specs']] == want.weight_specs
     assert len(want.weight_specs) > 200
@@ -178,18 +177,12 @@ def test_reference_backbone_builders_record_the_same_model():
     assert [tuple(s) for s in got['output_shape']] == [tuple(s) for s in want.output_shape]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 def test_reference_spnet_skeleton_records_the_same_model():
     """Same for deephar/models/spnet.py::entry_flow and models/common.py::residual_unit / downscaling_unit /
     upscaling_unit (the reference's code and its own ModelConfig / pose layout, on the recording keras)."""
     from deephar_b200 import common, spnet
     from deephar_b200.config import ModelConfig, pa16j2d
-    here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_backbone.py'), 'spnet'],
-                         capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0, out.stderr[-2000:]
-    got = json.loads([l for l in out.stdout.splitlines() if l.startswith('{')][-1])
+    got = _recorded('spnet')
     cfg = ModelConfig((256, 256, 3), pa16j2d, num_pyramids=2, num_levels=4, num_pose_features=160, num_visual_features=160)
     g = Graph('spnet_skeleton')
     x = spnet.entry_flow(g.input((256, 256, 3)), cfg)
@@ -203,8 +196,6 @@ def test_reference_spnet_skeleton_records_the_same_model():
     assert [tuple(s) for s in got['output_shape']] == [tuple(s) for s in want.output_shape]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 @pytest.mark.parametrize('concat', [0, 1])
 def test_reference_full_reception_build_records_the_headline_model(concat):
     """The reference's COMPLETE `reception.build()` (reception.py:225-321) -- unmodified file, Lambda channel slices
@@ -212,11 +203,7 @@ def test_reference_full_reception_build_records_the_headline_model(concat):
     builders taken from keras_compat: the recorded model IS deephar_b200.reception.build's (BASELINE configs[0]/[1]:
     weight list, auto-names, kernel plan, output order and shapes)."""
     from deephar_b200 import reception
-    here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_backbone.py'), 'full2d',
-                          str(concat)], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    got = json.loads([l for l in out.stdout.splitlines() if l.startswith('{')][-1])
+    got = _recorded('full2d %d' % concat)
     want = reception.build((256, 256, 3), 16, dim=2, num_context_per_joint=2, num_blocks=8, ksize=(5, 5),
                            concat_pose_confidence=bool(concat), export_heatmaps=bool(concat))
     assert [(n, tuple(s)) for n, s in got['weight_specs']] == want.weight_specs
@@ -225,12 +212,16 @@ def test_reference_full_reception_build_records_the_headline_model(concat):
     assert len(got['output_shape']) == 16        # 8 x (pose, visible), or 8 x (pose|visible, heat-maps)
 
 
-def _run_reference(*args):
-    here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_backbone.py')] + list(args),
-                         capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    lines = [json.loads(l) for l in out.stdout.splitlines() if l.startswith('{')]
+def _recorded_lines(case):
+    """The JSON lines tests/reference_dropin/run_reference_backbone.py printed for `case` (its arguments) when it ran the
+    reference's own builder code on the recording keras; stored by tests/golden/make_dropin_golden.py."""
+    with gzip.open(os.path.join(GOLDEN, 'ref_dropin_models.json.gz')) as f:
+        return json.load(f)[case]
+
+
+def _recorded(case):
+    """The recorded model of `case`, with the lines that follow it (split_model's) merged in."""
+    lines = _recorded_lines(case)
     got = next(d for d in lines if 'weight_specs' in d)
     for d in lines:
         if 'weight_specs' not in d:
@@ -253,22 +244,18 @@ def _same_model(got, want, same_launch_order=True):
     assert got['plan_checked'] > 2 * len(plan)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 def test_reference_reception_3d_build_records_the_c3_model():
     """reception.build(dim=3) of the reference, unmodified: the 3-D head is Lambda / keras.backend arithmetic there
     (reshape to (H, W, D, joints), two means, global max poolings, sigmoid -- reception.py:193-222); recorded as backend
     ops and rewritten into the fused pose_regression_3d op, the model is deephar_b200.reception.build's (BASELINE
     configs[2]), launch for launch."""
     from deephar_b200 import reception
-    got = _run_reference('full3d')
+    got = _recorded('full3d')
     want = reception.build((256, 256, 3), 17, dim=3, num_blocks=8, ksize=(5, 5), concat_pose_confidence=False)
     _same_model(got, want)
     assert len(got['plan']) == 134 and len(got['output_shape']) == 16
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 @pytest.mark.parametrize('which', ['penn', 'ntu'])
 def test_reference_full_spnet_build_records_the_c4_c5_models(which):
     """The reference's COMPLETE `spnet.build(cfg)` -- spnet.py, common.py, layers.py, activations.py, config.py, all
@@ -286,7 +273,7 @@ def test_reference_full_spnet_build_records_the_c4_c5_models(which):
     else:
         cfg = ModelConfig((16, 256, 256, 3), pa17j3d, num_actions=[60], num_pyramids=2, action_pyramids=[1, 2],
                           num_levels=4, pose_replica=False, num_pose_features=192, num_visual_features=192)
-    got = _run_reference('spnet_full', which)
+    got = _recorded('spnet_full ' + which)
     want = spnet.build(cfg)
     _same_model(got, want, same_launch_order=False)
     assert len(got['plan']) == {'penn': 345, 'ntu': 237}[which]
@@ -299,8 +286,6 @@ def test_reference_full_spnet_build_records_the_c4_c5_models(which):
     assert pshared and ashared              # views of the full model's network: the weights loaded into it are theirs
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 @pytest.mark.parametrize('pose_dim', [2, 3, 'v2'])
 def test_reference_merge_model_build_records_the_clip_models(pose_dim):
     """deephar/models/action.py::build_merge_model, unmodified, on the recording keras (SURVEY 8 a16 / f2): get_layer()
@@ -312,7 +297,7 @@ def test_reference_merge_model_build_records_the_clip_models(pose_dim):
     version = 'v1'
     if pose_dim == 'v2':                    # the wider PoseAR net (action.py:63-72), 2-D poses
         pose_dim, version = 2, 'v2'
-    got = _run_reference('merge', str(pose_dim), version)
+    got = _recorded('merge %d' % pose_dim + (' v2' if version == 'v2' else ''))
     if pose_dim == 2:
         pe = reception.build((256, 256, 3), 16, dim=2, num_blocks=4, num_context_per_joint=2, ksize=(5, 5))
         want = action.build_merge_model(pe, 15, (256, 256, 3), 16, 16, 4, pose_dim=2, pose_net_version=version)
@@ -323,26 +308,41 @@ def test_reference_merge_model_build_records_the_clip_models(pose_dim):
     assert len(got['weight_specs']) == 421 and len(got['output_shape']) == (9 if pose_dim == 2 else 11)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 def test_builder_options_off_the_baseline_configs_match_the_reference_builders():
     """reception.build / spnet.build arguments the BASELINE configs do not exercise (context maps 0 / 1, alpha, heat-map and
     feature export, depth_maps, 3 levels, growth, kernel 3x3, predict_rootz, several action sets, sam_alpha, image_div,
     other action pyramids, pa20j3d): the reference's builder, recorded, and the product's builder give the same model;
     what one refuses the other refuses."""
-    here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_backbone.py'), 'sweep'],
-                         capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stderr[-2000:]
-    rows = [json.loads(l) for l in out.stdout.splitlines() if l.startswith('{')]
-    assert len(rows) == 13
-    refused = [r for r in rows if 'ref_error' in r or 'prod_error' in r]
-    for r in refused:
-        assert 'ref_error' in r and 'prod_error' in r, r                   # never one side only
-    assert len(refused) == 3 and [r['ref_error'] for r in refused if r['tag'].startswith("reception {'dim': 4")] == ['ValueError']
-    for r in rows:
-        if r not in refused:
-            assert r['weights'] and r['signatures'] and r['shapes'] and r['launches'], r
+    from ref_cases import RECORDED_SWEEP_RECEPTION, RECORDED_SWEEP_SPNET, SWEEP_SPNET_BASE
+    from deephar_b200 import config as pconfig
+    from deephar_b200 import reception, spnet
+    rows = _recorded_lines('sweep')
+    assert len(rows) == len(RECORDED_SWEEP_RECEPTION) + len(RECORDED_SWEEP_SPNET) == 13
+    builders = []
+    for kw in RECORDED_SWEEP_RECEPTION:
+        nj = 17 if kw.get('dim') == 3 else 16
+        builders.append(('reception %r' % (kw,), lambda kw=kw, nj=nj: reception.build((128, 128, 3), nj, **kw)))
+    for shape, layout, extra in RECORDED_SWEEP_SPNET:
+        kw = dict(SWEEP_SPNET_BASE)
+        kw.update(extra)
+        builders.append(('spnet %r %s %r' % (shape, layout, extra),
+                         lambda shape=shape, layout=layout, kw=kw: spnet.build(pconfig.ModelConfig(shape, getattr(pconfig, layout), **kw))))
+    refused = 0
+    for ref, (tag, build) in zip(rows, builders):
+        assert ref['tag'] == tag
+        K.clear_session()
+        try:
+            prod = build()
+        except Exception as e:                                  # noqa: BLE001
+            assert ref.get('ref_error') == type(e).__name__, (tag, type(e).__name__)    # never one side only
+            refused += 1
+            continue
+        assert 'ref_error' not in ref, tag
+        assert [(n, tuple(s)) for n, s in ref['weight_specs']] == [(n, tuple(s)) for n, s in prod.weight_specs], tag
+        assert ref['signatures'] == prod.graph.signatures(), tag
+        assert [tuple(s) for s in ref['output_shape']] == [tuple(s) for s in prod.output_shape], tag
+        assert ref['kinds'] == sorted(k.kind for k in prod.plan.kops), tag
+    assert refused == 3 and [r['ref_error'] for r in rows if r['tag'].startswith("reception {'dim': 4")] == ['ValueError']
 
 
 def test_head_models_and_lambda_slices():
@@ -640,52 +640,60 @@ def test_a_model_of_some_outputs_shares_the_compiled_network():
     assert [n for n, _ in other.weight_specs] == ['a/kernel', 'b/kernel', 'c/kernel'] and other.optional_weights == ['b/kernel']
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 @pytest.mark.parametrize('which', ['mpii', 'h36m', 'penn_multitask', 'ntu_multitask', 'mpii+predict', 'h36m+predict'])
-def test_reference_entry_scripts_run_unmodified(tmp_path, which):
-    """The reference's entry scripts of every BASELINE config, executed AS THEY ARE (runpy) after dropin.install():
-    exp/mpii/eval_mpii_singleperson.py (configs[0]/[1], the headline model), exp/h36m/eval_h36m.py (configs[2]),
-    exp/pennaction/eval_penn_multitask.py (configs[3]) and exp/ntu/eval_ntu_multitask.py (configs[4]):
-    reception.build / spnet.build -> get_file (Keras cache look-up) / a local .hdf5 -> load_weights([by_name=True]) ->
-    the scripts' own re-wiring made after the weights were loaded (Model(model.input, [concatenate([pose, vis]) ...]),
-    split_model) -> the reference's own evaluators calling predict([x]) / predict(clip[None]).  The scores the evaluators
-    hand back to the script equal the ones recomputed from the oracle's outputs.  Stand-ins: datasets, checkpoint
-    contents and (no GPU here) the forward -- see tests/reference_dropin/run_reference_script.py.  The '+predict' variants
-    keep the product's OWN Model.predict / _bind / launch sequence under the evaluators and stand in only for the device
-    (tests/fake_cuda.py --arithmetic: numpy behind the C entry points)."""
+def test_reference_entry_scripts_run_unmodified(which):
+    """The reference's entry scripts of every BASELINE config, executed AS THEY ARE (runpy) after dropin.install()
+    (tests/reference_dropin/run_reference_script.py): exp/mpii/eval_mpii_singleperson.py (configs[0]/[1], the headline
+    model), exp/h36m/eval_h36m.py (configs[2]), exp/pennaction/eval_penn_multitask.py (configs[3]) and
+    exp/ntu/eval_ntu_multitask.py (configs[4]) -- reception.build / spnet.build, load_weights, the scripts' own re-wiring
+    (Model(model.input, [concatenate([pose, vis]) ...]), split_model) and the reference's own evaluators calling
+    predict().  What those runs ended up with is stored in tests/golden/ref_entry_scripts.json.gz
+    (make_entry_script_golden.py, which also checks there that the evaluators raised nothing): the scores the evaluators
+    returned and the recording of the re-wired model.  Here, without the reference, the same re-wiring is rebuilt with
+    keras_compat on deephar_b200's builders (tests/reference_dropin/standins.py): it records the same model (weights,
+    output expressions, launches, split views), holds the loaded weights, replays memory-safe and, executed on the CPU,
+    computes the oracle's outputs; and the scores recomputed from the oracle's outputs on the same stand-in datasets
+    equal the evaluators'.  The '+predict' variants recompute them from the product's OWN Model.predict / _bind / launch
+    sequence of the re-wired model, with only the device stood in for (tests/fake_cuda.py --arithmetic: numpy behind the
+    C entry points)."""
     here = os.path.dirname(os.path.abspath(__file__))
-    env = dict(os.environ, KERAS_HOME=str(tmp_path / 'keras'))
-    work = tmp_path / 'checkout'
-    work.mkdir()
+    with gzip.open(os.path.join(GOLDEN, 'ref_entry_scripts.json.gz')) as f:
+        rec = json.load(f)
     own_predict = which.endswith('+predict')
     which = which.split('+')[0]
-    cmd = [sys.executable, os.path.join(here, 'reference_dropin', 'run_reference_script.py'), which, str(work)]
+    rec = rec[which]
+    cmd = [sys.executable, os.path.join(here, 'reference_dropin', 'standins.py'), which]
     if own_predict:
-        env['DEEPHAR_B200_SCRIPT_ON_GPU'] = '1'
-        cmd = [sys.executable, os.path.join(here, 'fake_cuda.py'), '--arithmetic'] + cmd[1:]
-    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=env)
+        cmd = [sys.executable, os.path.join(here, 'fake_cuda.py'), '--arithmetic'] + cmd[1:] + ['predict']
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
     assert out.returncode == 0, out.stderr[-3000:]
-    assert 'exception on sample' not in out.stderr + out.stdout      # the multi-clip evaluators swallow predict() errors
     got = json.loads([l for l in out.stdout.splitlines() if l.startswith('{')][-1])
-    assert got['model_class'] == 'deephar_b200.keras_compat.Model'
-    assert got['weights_are_the_files']            # loaded BEFORE the re-wiring, shared with it as Keras shares layers
-    assert got['plan_checked'] > got['launches']   # the re-wired model's buffer plan replays memory-safe
-    assert got['plan_emulation_max_err'] < 5e-4    # ... and, executed on the CPU, computes the oracle's outputs (fp32 oracle)
     expected_calls = {'mpii': ['eval_singleperson_pckh'], 'h36m': ['eval_human36m_sc_error'],
                       'penn_multitask': ['eval_multiclip_dataset', 'eval_singleclip_generator', 'eval_singleperson_pckh'],
                       'ntu_multitask': ['eval_multiclip_dataset']}[which]
-    assert sorted(got['returned']) == sorted(got['oracle']) == expected_calls
+    assert sorted(rec['returned']) == sorted(got['returned']) == expected_calls
     for fn in expected_calls:
-        assert len(got['returned'][fn]) == 1
+        assert len(rec['returned'][fn]) == 1
         # fp32 buffers under the product's own predict vs the fp32 torch oracle: continuous scores agree to ~1e-6
-        assert got['returned'][fn][0] == pytest.approx(got['oracle'][fn][0], rel=1e-4 if own_predict else 1e-9, abs=1e-12), fn
-    assert got['forward'] == ('Model.predict' if own_predict else 'oracle (CPU stand-in)')
+        assert rec['returned'][fn][0] == pytest.approx(got['returned'][fn], rel=1e-4 if own_predict else 1e-9, abs=1e-12), fn
+    model = got['model']
+    for key in ('weight_specs', 'signatures', 'optional_weights', 'output_shape'):
+        assert model[key] == rec['model'][key], key
+    # the same launches; in the same order except for SPNet's per-block pose-output copies (as in
+    # test_reference_full_spnet_build_records_the_c4_c5_models)
+    assert sorted(map(str, model['plan'])) == sorted(map(str, rec['model']['plan']))
     if which in ('mpii', 'h36m'):
-        assert got['output_shape'] == [[None, 16 if which == 'mpii' else 17, 3 if which == 'mpii' else 4]] * 8
+        assert model['plan'] == rec['model']['plan']
+    assert got['split'] == rec['split']
+    assert model['weights_are_the_files']            # loaded BEFORE the re-wiring, shared with it as Keras shares layers
+    assert model['plan_checked'] > model['launches']   # the re-wired model's buffer plan replays memory-safe
+    assert model['plan_emulation_max_err'] < 5e-4    # ... and, executed on the CPU, computes the oracle's outputs (fp32 oracle)
+    if which in ('mpii', 'h36m'):
+        assert rec['output_shape'] == [[None, 16 if which == 'mpii' else 17, 3 if which == 'mpii' else 4]] * 8
     else:
-        assert got['output_shape'] == [[None, 15 if which == 'penn_multitask' else 60]] * 6      # the 'Action' split
-        assert max(got['returned']['eval_multiclip_dataset'][0]) == 50.0        # labels: one right, one wrong by design
+        assert rec['output_shape'] == [[None, 15 if which == 'penn_multitask' else 60]] * 6      # the 'Action' split
+        assert [s[3] for s in rec['split']] == [True, True]          # views of the loaded full network
+        assert max(rec['returned']['eval_multiclip_dataset'][0]) == 50.0        # labels: one right, one wrong by design
 
 
 def test_get_file_is_a_cache_lookup(tmp_path, monkeypatch):

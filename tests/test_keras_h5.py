@@ -39,12 +39,10 @@ def test_hdf5_roundtrip_types_and_big_groups(tmp_path):
 
 
 def test_reads_a_file_written_by_libhdf5():
-    """The only real libhdf5 output in the image: scipy's MATLAB v7.3 test file (512-byte user block,
-    old-style groups, v1 object headers, attributes)."""
-    scipy_io = pytest.importorskip('scipy.io')
-    path = os.path.join(os.path.dirname(scipy_io.__file__), 'matlab', 'tests', 'data', 'testhdf5_7.4_GLNX86.mat')
-    if not os.path.exists(path):
-        pytest.skip('scipy test data not installed')
+    """A file libhdf5 wrote: MATLAB v7.3 output from SciPy's test data, stored as tests/golden/testhdf5_7.4_GLNX86.mat
+    (source and licence: testhdf5_7.4_GLNX86.mat.LICENSE beside it) -- 512-byte user block, old-style groups, v1 object
+    headers, attributes."""
+    path = os.path.join(HERE, 'golden', 'testhdf5_7.4_GLNX86.mat')
     with hdf5.File(path) as f:
         assert f.keys() == ['testdouble']
         d = f['testdouble']

@@ -2,7 +2,7 @@
 
 tests/golden/ref_*.npz were written by tests/golden/make_reference_golden.py, which imports
 deephar/models/{reception,spnet,action,blocks,common}.py, layers.py and activations.py UNMODIFIED from
-/root/reference and executes them on tests/golden/keras_shim (an eager float64 stand-in for the Keras 2.1.4
+the reference checkout and executes them on tests/golden/keras_shim (an eager float64 stand-in for the Keras 2.1.4
 API; keras/tensorflow themselves are not installable here).  Each fixture holds the weight list of the
 reference model as Keras would save it, and the outputs of the reference graph for seeded inputs and the
 product's synthetic weights (assigned by name).
@@ -216,19 +216,39 @@ def test_product_matches_reference_graph(cuda, case):
         assert ties <= max(1, maps // 20), '%d of %d heat-maps have an unresolvable top-2 tie' % (ties, maps)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get('DEEPHAR_REFERENCE', '/root/reference')),
-                    reason='needs the reference tree (development container only)')
 def test_options_off_the_baseline_configs_numerically():
-    """Live, no stored fixture: for builder arguments the BASELINE configs do not use (no / one context map, alpha,
-    heat-map and feature export, depth_maps, 3 pyramid levels, growth, 3x3 kernels, predict_rootz, two action sets,
-    sam_alpha, image_div, pa20j3d, other action pyramids) the reference's own builder code is executed on the eager
-    float64 Keras shim and compared with the product's compiled plan executed by tests/plan_emulator.py."""
-    import json
-    import subprocess
-    out = subprocess.run([sys.executable, os.path.join(HERE, 'golden', 'run_option_sweep_numeric.py')],
-                         capture_output=True, text=True, timeout=1500)
-    assert out.returncode == 0, out.stderr[-3000:]
-    rows = [json.loads(l) for l in out.stdout.splitlines() if l.startswith('{')]
-    assert len(rows) == 10
-    for r in rows:
-        assert r['max_rel_err'] <= 1e-9, r
+    """For builder arguments the BASELINE configs do not use (no / one context map, alpha, heat-map and feature export,
+    depth_maps, 3 pyramid levels, growth, 3x3 kernels, predict_rootz, two action sets, sam_alpha, image_div, pa20j3d,
+    other action pyramids): the product's compiled plan, executed by tests/plan_emulator.py, reproduces the outputs of the
+    reference's own builder code executed on the eager float64 Keras shim (tests/golden/ref_option_sweep.npz, written by
+    make_option_sweep_golden.py) for the same seeded inputs and synthetic weights."""
+    import zlib
+    from plan_emulator import PlanEmulator
+    from ref_cases import option_sweep_inputs, option_sweep_sample_index
+    from deephar_b200 import config as pconfig
+    z = np.load(os.path.join(HERE, 'golden', 'ref_option_sweep.npz'))
+    cases = option_sweep_inputs()
+    assert len(cases) == 10
+    for i, (kind, spec, x) in enumerate(cases):
+        if kind == 'reception':
+            m = reception.build((64, 64, 3), 17 if spec['dim'] == 3 else 16, **spec)
+        else:
+            shape, layout, kw = spec
+            m = spnet.build(pconfig.ModelConfig(shape, getattr(pconfig, layout), **kw))
+        assert zlib.crc32(np.ascontiguousarray(x, dtype=np.float32).tobytes()) == int(z['x_crc32_%d' % i]), \
+            'regenerated input differs from the one the fixture was made with'
+        optional = set(m.optional_weights)
+        assert sorted(n for n, _ in m.weight_specs if n not in optional) == [str(n) for n in z['names%d' % i]], (i, spec)
+        m.init_synthetic_weights(1234)
+        with np.errstate(over='ignore'):
+            outs = PlanEmulator(m).run(x)
+        assert len(outs) == len({f.split('_')[1] for f in z.files if f.startswith('out%d_' % i)}), (i, spec)
+        for k, o in enumerate(outs):
+            key = 'out%d_%d' % (i, k)
+            if key in z.files:
+                r = z[key]
+                assert o.shape == r.shape, (i, spec, k)
+            else:                   # a large output: its shape and the values at fixed positions
+                assert o.shape == tuple(z[key + '_shape']), (i, spec, k)
+                o, r = o.ravel()[option_sweep_sample_index(o.size)], z[key + '_sample']
+            assert np.abs(o - r).max() <= 1e-9 * max(1.0, np.abs(r).max()), (i, spec, k, float(np.abs(o - r).max()))
